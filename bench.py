@@ -20,6 +20,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -175,7 +176,8 @@ class CpuArm:
     def __init__(self, snap):
         from oracle import oracle
         self.oracle = oracle
-        self.L = oracle.load(oracle.build_native())
+        self._tmp = tempfile.TemporaryDirectory(prefix="kr_oracle_native_")  # the tree may be read-only
+        self.L = oracle.load(oracle.build_native(self._tmp.name))
         t0 = time.perf_counter()
         self.cx = oracle.Context(snap, self.L)
         self.ctx_build_ms = 1e3 * (time.perf_counter() - t0)
@@ -201,6 +203,38 @@ class CpuArm:
 
     def close(self):
         self.cx.close()
+        self._tmp.cleanup()
+
+
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(res, out_dir: str) -> None:
+    """--dump-outputs: the records one pass hands its caller, one float array per field as out_dir/<name>.npy (8-bit fields as
+    float32, wider ones as float64: both exact).  The two variable-length lists are written in owner order (each RayCluster's
+    actions, each group's replica indices), without their arena offsets, which are layout rather than results.  An array with
+    no rows is not written (a workload without RayJobs has no jobs.* records).  Above DUMP_CAP_BYTES in all, every array keeps
+    the same fixed, seeded sample of the same fraction of its rows."""
+    from kuberay_b200.abi import _gather_owned
+    arrays = {}
+    for rec in ("clusters", "groups", "jobs"):
+        a = getattr(res, rec)
+        for f in a.dtype.names:
+            if f not in ("create_off", "reserved"):
+                arrays[f"{rec}.{f}"] = a[f]
+    arrays.update(hash=res.hash, wtd_pod_idx=res.wtd_pod_idx, act_cnt=res.act_cnt)
+    acts = _gather_owned(res.act_start[:-1], res.act_cnt)
+    arrays.update(act_pod_idx=res.act_pod_idx[acts], act_code=res.act_code[acts],
+                  create_idx=res.create_idx[_gather_owned(res.groups["create_off"], res.groups["n_create"])])
+    arrays = {k: v.astype(np.float32 if v.dtype.itemsize == 1 else np.float64) for k, v in arrays.items() if len(v)}
+    frac = DUMP_CAP_BYTES / sum(v.nbytes for v in arrays.values())
+    if frac < 1:
+        for k, v in arrays.items():
+            arrays[k] = v[np.sort(np.random.default_rng(0).choice(len(v), max(1, int(len(v) * frac)), replace=False))]
+    arrays["totals"] = np.array([res.n_create_total, res.n_orphans, res.n_actions], dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def run_reference(args, rank: int, world: int):
@@ -246,6 +280,7 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"], help="weak: the workload per GPU (default); strong: the workload once, split over the GPUs")
     ap.add_argument("--no-pack-leg", action="store_true", help="skip the e2e_with_pack leg (tools/pack_bench)")
     ap.add_argument("--no-next-rows", action="store_true", help="skip the f2-f4 extras (tools/f4_bench.py, tools/f3_bench.py --quick)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of the last timed step of the value leg (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -324,6 +359,7 @@ def main():
         dev_ms += step_device()
     barrier()
     wall_ms = 1e3 * (time.perf_counter() - wall0)
+    last_step = eng.fetch() if args.dump_outputs and rank == 0 else None
     n_kernels = eng.last_profile()["n_kernels"]
     # the same graph without the hash kernel: the match -> decide chain on its own (what pipeline_roofline is quoted on)
     flags.skip_hash = 1
@@ -601,6 +637,8 @@ def main():
                 "all_threads_indexed_lists": {"value": vi, "unit": UNIT, "cores": threads, "sample": f"{si} reconciles in {di:.1f} s (pods pre-bucketed by cluster: no namespace scan)"}}
             arm.close()
         os.write(json_fd, (json.dumps(line) + "\n").encode())
+        if last_step is not None:
+            dump_outputs(last_step, args.dump_outputs)
     eng.close()
     if world > 1:
         dist.destroy_process_group()

@@ -27,10 +27,11 @@ def build(force: bool = False) -> str:
     return so
 
 
-def build_native() -> str:
-    """The CPU arm's build: same source, -O3 -march=native for the host it runs on (bench.py only; never shipped)."""
-    subprocess.check_call(["make", "-s", "-C", _HERE, "-B", "libkroracle_native.so"])
-    return os.path.join(_HERE, "libkroracle_native.so")
+def build_native(out_dir: str) -> str:
+    """The CPU arm's build: same source, -O3 -march=native for the host it runs on, into out_dir (bench.py only; never shipped)."""
+    so = os.path.join(out_dir, "libkroracle_native.so")
+    subprocess.check_call(["make", "-s", "-C", _HERE, "-B", "native", "NATIVE=" + so])
+    return so
 
 
 def _bind(L: C.CDLL) -> C.CDLL:

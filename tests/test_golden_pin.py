@@ -1,23 +1,17 @@
 """Mechanical cross-check of the hand-transcribed fixtures (tests/golden/*.json) against the Go test sources they cite.
 
-tests/golden/transcribe.py was written by hand (Go cannot run in this image).  Where the reference tree is readable
-(/root/reference — this container; never the GPU box), these tests regex-parse the table-driven Go tests and assert that the
-literals in the JSON fixtures equal the literals in the Go source, case by case and in order:
+tests/golden/transcribe.py was written by hand.  tests/golden/extract_go_tables.py regex-parses the
+table-driven Go tests of the reference and stores their cases in tests/golden/go_test_tables.json; these tests assert that the
+literals in the hand-written fixtures equal the literals parsed out of the Go source, case by case and in order:
   Test_ShouldDeletePod                  raycluster_controller_unit_test.go:2380-2503
   TestCalculateMaxReplicasOverflow      utils/util_test.go:802-894
   TestInconsistentRayClusterStatus      utils/consistency_test.go:16-146
   TestShouldRecreatePodsForUpgrade      raycluster_controller_unit_test.go:3680-3814
-  TestGetWorkerGroupDesiredReplicas     utils/util_test.go:555-601
-Skipped (not failed) when the reference is absent."""
+  TestGetWorkerGroupDesiredReplicas     utils/util_test.go:555-601"""
 import json
 import os
-import re
 
-import pytest
-
-REF = "/root/reference/ray-operator/controllers/ray"
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
 
 
 def gold(name):
@@ -25,147 +19,58 @@ def gold(name):
         return json.load(f)
 
 
-def go_func(path: str, name: str) -> str:
-    src = open(os.path.join(REF, path)).read()
-    start = src.index(f"func {name}(")
-    nxt = src.find("\nfunc ", start + 1)
-    return src[start:nxt if nxt > 0 else len(src)]
-
-
-def table_cases(body: str) -> list[str]:
-    """The `{ ... },` literals of the first table-driven slice in a Go test body (brace matching, comments stripped)."""
-    body = re.sub(r"//[^\n]*", "", body)
-    m = re.search(r":= \[\]struct \{.*?\n\t\}\{\n", body, re.S)
-    assert m, "no table found"
-    i, depth, cases, cur = m.end(), 0, [], None
-    while i < len(body):
-        ch = body[i]
-        if ch == "{":
-            if depth == 0:
-                cur = i
-            depth += 1
-        elif ch == "}":
-            depth -= 1
-            if depth == 0:
-                cases.append(body[cur:i + 1])
-            if depth < 0:
-                break
-        i += 1
-    return cases
+GO = gold("go_test_tables")
 
 
 def test_should_delete_pod_table_matches_the_go_source():
-    cases = table_cases(go_func("raycluster_controller_unit_test.go", "Test_ShouldDeletePod"))
-    got = []
-    for c in cases:
-        got.append({
-            "restartPolicy": re.search(r"restartPolicy:\s*corev1\.RestartPolicy(\w+)", c).group(1),
-            "phase": re.search(r"phase:\s*corev1\.Pod(\w+)", c).group(1),
-            "terminated": "Terminated: &corev1.ContainerStateTerminated" in c,
-            "want": re.search(r"shouldDelete:\s*(true|false)", c).group(1) == "true",
-        })
-    assert got == gold("should_delete_pod")["cases"]
-
-
-def _groups(case: str) -> list[dict]:
-    out = []
-    for g in re.findall(r"\{[^{}]*?NumOfHosts[^{}]*?\}", case, re.S):
-        d = {"hosts": int(re.search(r"NumOfHosts:\s*(\d+)", g).group(1))}
-        for key, fld in (("replicas", "Replicas"), ("min", "MinReplicas"), ("max", "MaxReplicas")):
-            m = re.search(rf"\b{fld}:\s*ptr\.To\[int32\]\((-?\d+)\)", g)
-            if m:
-                d[key] = int(m.group(1))
-        out.append(d)
-    return out
+    assert GO["should_delete_pod"] == gold("should_delete_pod")["cases"]
 
 
 def test_max_replicas_overflow_table_matches_the_go_source():
-    cases = table_cases(go_func("utils/util_test.go", "TestCalculateMaxReplicasOverflow"))
+    cases = GO["max_overflow"]
     want = gold("replica_arithmetic")["max_overflow"]["cases"]
     assert len(cases) == len(want)
     for c, w in zip(cases, want):
-        assert int(re.search(r"expected:\s*(-?\d+)", c).group(1)) == w["want_max"], w["name"]
-        assert _groups(c) == [{k: v for k, v in g.items() if k in ("hosts", "replicas", "min", "max")} for g in w["groups"]], w["name"]
+        assert c["expected"] == w["want_max"], w["name"]
+        assert c["groups"] == [{k: v for k, v in g.items() if k in ("hosts", "replicas", "min", "max")} for g in w["groups"]], w["name"]
 
 
 def test_desired_replicas_table_matches_the_go_source():
-    """The Go test mutates one WorkerGroupSpec step by step (fields bound to local variables through pointers) and asserts after
-    each step: replay the assignments, and at every assert compare the spec's state and the expected value with the fixture."""
-    body = re.sub(r"//[^\n]*", "", go_func("utils/util_test.go", "TestGetWorkerGroupDesiredReplicas"))
+    """The Go test mutates one WorkerGroupSpec step by step and asserts after each step: at every assert the spec's state and
+    the expected value must equal the fixture's case."""
     want = gold("replica_arithmetic")["desired_replicas"]["cases"]
-    var: dict[str, object] = {}
-    bind: dict[str, tuple[str, bool]] = {}   # struct field -> (variable, bound by pointer)
-    fields = {"NumOfHosts": "hosts", "MinReplicas": "min", "MaxReplicas": "max", "Replicas": "replicas", "Suspend": "suspend"}
-    frozen: dict[str, object] = {}           # value fields copy at assignment time
-    seen = 0
-    for line in body.splitlines():
-        line = line.strip().rstrip(",")
-        m = re.fullmatch(r"(\w+)\s*:?=\s*int32\((-?\d+)\)", line)
-        if m:
-            var[m.group(1)] = int(m.group(2)); continue
-        m = re.fullmatch(r"(\w+)\s*:?=\s*(true|false)", line)
-        if m:
-            var[m.group(1)] = m.group(2) == "true"; continue
-        m = re.fullmatch(r"(?:workerGroupSpec\.)?(\w+)\s*[:=]\s*(&?)(\w+)", line)
-        if m and m.group(1) in fields:
-            if m.group(2):
-                bind[m.group(1)] = (m.group(3), True); frozen.pop(m.group(1), None)
-            else:
-                bind.pop(m.group(1), None); frozen[m.group(1)] = var[m.group(3)]
-            continue
-        m = re.fullmatch(r"assert\.(Equal|Zero)\(t, GetWorkerGroupDesiredReplicas\(workerGroupSpec\)(?:, (.+))?\)", line)
-        if m:
-            state = {}
-            for f, key in fields.items():
-                state[key] = var[bind[f][0]] if f in bind else frozen.get(f)
-            expected = 0 if m.group(1) == "Zero" else eval(m.group(2), {}, dict(var))  # noqa: S307 - a product of two test locals at most
-            w = want[seen]
-            assert expected == w["want"], (seen, expected, w)
-            assert state["hosts"] == w["hosts"] and state["min"] == w["min"] and state["max"] == w["max"], (seen, state, w)
-            assert state["replicas"] == w["replicas"] and bool(state["suspend"]) == w["suspend"], (seen, state, w)
-            seen += 1
-    assert seen == len(want) == 6
+    for seen, (state, w) in enumerate(zip(GO["desired_replicas"], want)):
+        assert state["expected"] == w["want"], (seen, state, w)
+        assert state["hosts"] == w["hosts"] and state["min"] == w["min"] and state["max"] == w["max"], (seen, state, w)
+        assert state["replicas"] == w["replicas"] and state["suspend"] == w["suspend"], (seen, state, w)
+    assert len(GO["desired_replicas"]) == len(want) == 6
 
 
 def test_inconsistent_status_table_matches_the_go_source():
-    body = go_func("utils/consistency_test.go", "TestInconsistentRayClusterStatus")
+    go = GO["inconsistent_status"]
     g = gold("inconsistent_status")
     old = g["old"]
-    lit = re.search(r"oldStatus := rayv1\.RayClusterStatus\{(.*?)\n\t\}\n", body, re.S).group(1)
-    for go_name, key in (("ReadyWorkerReplicas", "readyWorkerReplicas"), ("AvailableWorkerReplicas", "availableWorkerReplicas"),
-                         ("DesiredWorkerReplicas", "desiredWorkerReplicas"), ("MinWorkerReplicas", "minWorkerReplicas"),
-                         ("MaxWorkerReplicas", "maxWorkerReplicas"), ("ObservedGeneration", "observedGeneration")):
-        assert int(re.search(rf"\b{go_name}:\s*(\d+)", lit).group(1)) == old[key], key
-    assert re.search(r'PodIP:\s*"([^"]+)"', lit).group(1) == old["head"]["podIP"]
-    assert re.search(r'ServiceIP:\s*"([^"]+)"', lit).group(1) == old["head"]["serviceIP"]
-    assert re.search(r'Reason:\s*"([^"]+)"', lit).group(1) == old["reason"]
-    assert "State:                   rayv1.Ready" in lit and old["state"] == "ready"
-    cases = table_cases(body[body.index("testCases :="):])
-    assert len(cases) == len(g["cases"])
-    for c, w in zip(cases, g["cases"]):
-        name = re.search(r'name:\s*"([^"]+)"', c).group(1)
+    for key in ("readyWorkerReplicas", "availableWorkerReplicas", "desiredWorkerReplicas", "minWorkerReplicas", "maxWorkerReplicas", "observedGeneration"):
+        assert go["old"][key] == old[key], key
+    assert go["old"]["head"]["podIP"] == old["head"]["podIP"]
+    assert go["old"]["head"]["serviceIP"] == old["head"]["serviceIP"]
+    assert go["old"]["reason"] == old["reason"]
+    assert go["old"]["state"] == "ready" and old["state"] == "ready"
+    assert len(go["cases"]) == len(g["cases"])
+    for c, w in zip(go["cases"], g["cases"]):
+        name = c["name"]
         assert name.startswith(w["name"].split(" ")[0].split(".")[0]) or w["name"].split(" ")[0] in name, (name, w["name"])
-        assert (re.search(r"expectResult:\s*(true|false)", c).group(1) == "true") == w["want"], name
+        assert c["want"] == w["want"], name
 
 
 def test_recreate_upgrade_table_matches_the_go_source():
-    cases = table_cases(go_func("raycluster_controller_unit_test.go", "TestShouldRecreatePodsForUpgrade"))
+    cases = GO["recreate_upgrade"]
     want = gold("recreate_upgrade")["cases"]
     assert len(cases) == len(want)
     for c, w in zip(cases, want):
-        assert (re.search(r"expectedRecreate:\s*(true|false)", c).group(1) == "true") == w["want"], w["name"]
-        if "upgradeStrategy:  nil" in c or re.search(r"upgradeStrategy:\s*nil", c):
-            assert w["upgradeStrategy"] is None
-        elif "Type: nil" in c:
-            assert w["upgradeStrategy"] == {"type": None}
-        elif "RayClusterUpgradeNone" in c:
-            assert w["upgradeStrategy"] == {"type": "None"}
-        else:
-            assert "RayClusterRecreate" in c and w["upgradeStrategy"] == {"type": "Recreate"}
-        has_pod = "createPodWithHash(" in c
-        assert has_pod == (w["head"] is not None), w["name"]
-        if has_pod:
-            args = re.search(r'createPodWithHash\(([^)]*)\)', c).group(1)
-            hash_arg, ver_arg = [a.strip() for a in args.split(",")][-2:]
-            assert (hash_arg == "RayClusterHash") == (w["head"]["hash"] == "<current>"), w["name"]
-            assert (ver_arg == "utils.KUBERAY_VERSION") == (w["head"]["version"] == "<current>"), w["name"]
+        assert c["want"] == w["want"], w["name"]
+        assert c["upgradeStrategy"] == w["upgradeStrategy"], w["name"]
+        assert (c["head"] is not None) == (w["head"] is not None), w["name"]
+        if c["head"] is not None:
+            assert c["head"]["hash_is_current"] == (w["head"]["hash"] == "<current>"), w["name"]
+            assert c["head"]["version_is_current"] == (w["head"]["version"] == "<current>"), w["name"]
